@@ -2,7 +2,7 @@
 """bench.py — edges/s for forward+backward of the layer of one BASELINE.json config, with the HBM roofline of its dominant
 kernel, the reference's CPU path timed beside it, parity against the oracle and an end-to-end number on host buffers.
 
-    python bench.py [--config 1..5] [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--config 1..5] [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Default (what the driver runs): config 2 = BASELINE configs[1], the config the metric is quoted on — one GCNConv 128->128
 (add_self_loops, relu, bias) forward + backward on RMAT N = 10 M, E = 100 M, fp32.
@@ -19,6 +19,11 @@ Default (what the driver runs): config 2 = BASELINE configs[1], the config the m
             same workload, timed on the host cores; the GPU runs the same sample and the two results are compared.
 `--impl reference`: the reference's CPU path (oracle port; Julia cannot run here) at the FULL size of the config when the
             host has the memory (config 2: ~60 GB), else the bounded sample (says which).
+`--dump-outputs DIR`: after the timed steps of config 2, what the last step returned to its caller (y, dx, dW, db) as
+            DIR/<name>.npy, float32; the row arrays as the same seeded sample of rows (row_ids.npy), under 64 MB in all.
+            The inputs are seeded, so two builds run with the same arguments can be compared output for output.
+
+bench.py writes nothing into the tree it runs from (the tree may be read-only): no bytecode caches either.
 """
 import argparse
 import json
@@ -28,9 +33,11 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 SEED = 17
+DUMP_BYTES = 60_000_000          # array data of --dump-outputs; the .npy headers add 128 bytes a file
 
 # BASELINE.json configs (SURVEY.md §8: sizes BASELINE leaves open are this project's choice, stated with every number)
 CFG = {
@@ -61,7 +68,13 @@ def parse():
     ap.add_argument("--no-parity", action="store_true", help="skip the full-size parity check of the partitioned path (debug)")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer leg (debug)")
     ap.add_argument("--ref-sample", action="store_true", help="--impl reference on the bounded sample instead of the full size")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (config 2, one GPU)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and (a.config != 2 or a.impl != "ours"):
+        ap.error("--dump-outputs is written by the GPU run of config 2")
     c = CFG[a.config]
     a.nodes = a.nodes or c["nodes"]
     a.edges = a.edges or c["edges"]
@@ -401,6 +414,24 @@ def make_flush(torch, dev):
     return lambda: buf.zero_()
 
 
+def dump_outputs(out_dir, rows, whole, n):
+    """Write `whole` (name -> tensor) in full and `rows` (name -> tensor with n rows) on one fixed, seeded sample of rows,
+    listed in row_ids.npy, as out_dir/<name>.npy in float32; all rows when they fit DUMP_BYTES."""
+    import numpy as np
+    import torch
+    room = DUMP_BYTES - sum(4 * v.numel() for v in whole.values())
+    k = min(n, room // (8 + sum(4 * v[0].numel() for v in rows.values())))
+    if k < 1:
+        raise SystemExit(f"--dump-outputs: the outputs do not fit {DUMP_BYTES} bytes")
+    ids = np.arange(n) if k == n else np.sort(np.random.default_rng(SEED).choice(n, k, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "row_ids.npy"), ids.astype(np.float64))
+    for name, v in rows.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), v[torch.as_tensor(ids, device=v.device)].float().cpu().numpy())
+    for name, v in whole.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), v.float().cpu().numpy())
+
+
 def base_line(args, value, ms, n_gpus, workload, extra_cfg, clocks, e2e, launches, roof, cpu, parity, dtype="f32"):
     cfg = {"workload": workload}
     cfg.update(extra_cfg)
@@ -430,9 +461,11 @@ def run_config2(args, torch, gnn, dev):
     t_plan = time.perf_counter() - t0
 
     gen = torch.Generator(device=dev).manual_seed(0)
+    torch.manual_seed(0)                    # the weights: torch seeds its CUDA generators differently in every process
     layer = gnn.GCNConv(D, D, torch.relu, device=dev)
     x = gnn.unrows(torch.randn(n, D, device=dev, generator=gen)).requires_grad_(True)
     dy = gnn.unrows(torch.randn(n, D, device=dev, generator=gen))
+    last = {}
 
     def step():
         x.grad = None
@@ -440,6 +473,8 @@ def run_config2(args, torch, gnn, dev):
         layer.bias.grad = None
         y = layer(g, x)
         y.backward(dy)
+        if args.dump_outputs:
+            last["y"] = y
         return y
 
     for _ in range(args.warmup):
@@ -449,6 +484,9 @@ def run_config2(args, torch, gnn, dev):
     ms, clocks = timed_region(torch, step, args.steps, dev, dev.index or 0)
     launches = gnn.launch_count() - l0
     value = E / (ms * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"y": gnn.rows(last.pop("y").detach()), "dx": gnn.rows(x.grad)},
+                     {"dW": layer.weight.grad, "db": layer.bias.grad}, n)
 
     # ---- the dominant kernel alone: fused GCN propagate (both directions), CUDA events on the launch stream
     xr = gnn.rows(x.detach())
@@ -931,6 +969,8 @@ def run_ours(args):
     torch.backends.cuda.matmul.allow_tf32 = False   # fp32 GEMM like the reference (cuBLAS sgemm)
     torch.backends.cudnn.allow_tf32 = False
     if world > 1 or os.environ.get("GNNB_BENCH_PARTITIONED"):   # the env switch: the partitioned path on one rank (debug)
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs is written by the single-GPU path")
         dist.init_process_group("nccl", device_id=dev)
         if args.config not in (2, 5):
             raise SystemExit("configs 1, 3, 4 are single-GPU workloads")

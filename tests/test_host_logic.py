@@ -1,6 +1,7 @@
 """Host-side mirror of the reference interface: size checks, containers, layout helpers, batching.
 CPU only (no kernels run)."""
 import operator
+import sys
 
 import numpy as np
 import pytest
@@ -167,3 +168,40 @@ def test_bench_argument_surface():
     assert (a.gpus, a.steps, a.warmup, a.config) == (8, 4, 3, 5)
     assert a.no_parity and a.no_cpu and a.no_e2e and a.impl != "reference"
     assert (a.nodes, a.edges, a.dim) == (100_000_000, 1_000_000_000, 256)     # config 5 = BASELINE configs[4]
+
+
+def test_bench_dump_outputs_and_its_arguments(tmp_path, monkeypatch):
+    """--dump-outputs: float32 files, one seeded row sample shared by the row arrays and the same on every call, the
+    whole budget respected; all rows when they fit.  --steps must be a real count."""
+    b = _bench_module()
+    n, D = 1000, 3
+    g = torch.Generator().manual_seed(0)
+    y, dx = torch.randn(n, D, generator=g), torch.randn(n, D, generator=g)
+    dW, db = torch.randn(D, D, generator=g), torch.randn(D, generator=g)
+    monkeypatch.setattr(b, "DUMP_BYTES", 8000)
+    for d in ("a", "b"):
+        b.dump_outputs(str(tmp_path / d), {"y": y, "dx": dx}, {"dW": dW, "db": db}, n)
+    got = {f.stem: np.load(f) for f in (tmp_path / "a").glob("*.npy")}
+    assert sorted(got) == ["dW", "db", "dx", "row_ids", "y"]
+    assert all(v.dtype == (np.float64 if k == "row_ids" else np.float32) for k, v in got.items())
+    ids = got["row_ids"].astype(np.int64)
+    assert 100 < len(ids) < n and (np.diff(ids) > 0).all() and ids[-1] < n
+    assert np.array_equal(got["y"], y.numpy()[ids]) and np.array_equal(got["dx"], dx.numpy()[ids])
+    assert np.array_equal(got["dW"], dW.numpy()) and np.array_equal(got["db"], db.numpy())
+    assert sum(v.nbytes for v in got.values()) <= 8000
+    for k, v in got.items():
+        assert np.array_equal(np.load(tmp_path / "b" / f"{k}.npy"), v)
+    monkeypatch.setattr(b, "DUMP_BYTES", 60_000_000)
+    b.dump_outputs(str(tmp_path / "c"), {"y": y}, {}, n)
+    assert np.array_equal(np.load(tmp_path / "c" / "row_ids.npy"), np.arange(n))
+    monkeypatch.setattr(b, "DUMP_BYTES", 10)
+    with pytest.raises(SystemExit):
+        b.dump_outputs(str(tmp_path / "d"), {"y": y}, {"dW": dW}, n)
+    for argv in (["--steps", "0"], ["--warmup", "-1"], ["--config", "3", "--dump-outputs", str(tmp_path)],
+                 ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        monkeypatch.setattr(sys, "argv", ["bench.py"] + argv)
+        with pytest.raises(SystemExit):
+            b.parse()
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--gpus", "1", "--steps", "7", "--warmup", "2", "--dump-outputs", "out"])
+    a = b.parse()
+    assert (a.steps, a.warmup, a.dump_outputs, a.config) == (7, 2, "out", 2)
