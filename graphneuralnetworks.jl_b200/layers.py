@@ -337,9 +337,14 @@ class _GATCoreFn(torch.autograd.Function):
 
 
 def gat_logit_fusable(chout: int, heads: int) -> bool:
-    """shapes csrc/gatlogit.cu covers: C/4 a power of two <= 32, C*H <= 4096 (config 3: 64 x 8)"""
+    """Shapes both gnnb_gat_logit_terms and gnnb_gat_logit_terms_bwd (csrc/gatlogit.cu) cover: G = C/4 a power of two <= 32,
+    C*H <= 4096, at most 8 passes of 32/G heads per warp, and a block stage of 8 warps x 2*H*C floats = 64*H*C bytes
+    <= 200 KiB (config 3, 64 x 8: 4 passes of 2 heads, 32 KiB).  Other shapes take the el / er broadcasts."""
     g = chout // 4
-    return chout % 4 == 0 and g > 0 and (g & (g - 1)) == 0 and g <= 32 and chout * heads <= 4096 and (heads * 4 + chout // 4 - 1) // (chout // 4) <= 64
+    if not (heads >= 1 and chout % 4 == 0 and g > 0 and (g & (g - 1)) == 0 and g <= 32 and chout * heads <= 4096):
+        return False
+    passes = -(-heads // (32 // g))
+    return passes <= 8 and 64 * heads * chout <= 200 * 1024
 
 
 def gat_fusable(chout: int, heads: int) -> bool:

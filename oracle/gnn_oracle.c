@@ -9,7 +9,8 @@
  *   GNNlib/src/msgpass.jl:71-79,117-129,145-149,191-208,215-238   propagate / apply_edges / aggregate_neighbors
  *   GNNGraphs/src/gatherscatter.jl:1-18                            _gather / _scatter -> NNlib.gather / scatter
  *   GNNlib/src/utils.jl:84-97                                      softmax_edge_neighbors
- *   GNNlib/src/layers/conv.jl:14-72,112-167,277-283                gcn_conv / gat_conv / sage_conv (edge parts)
+ *   GNNlib/src/layers/conv.jl:14-72,112-167,277-283                gcn_conv / gat_conv / sage_conv (edge parts;
+ *                                                                  gat_conv's also in closed-form pullback)
  *   GNNGraphs/src/query.jl:220-231,314-369                         adjacency_matrix / degree
  *   GNNGraphs/src/convert.jl:221-237                               to_sparse (COO -> CSC, duplicates summed)
  * The arithmetic itself lives in a third-party dependency that is NOT in the reference tree:

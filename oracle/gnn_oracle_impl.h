@@ -225,3 +225,56 @@ int FN(orc_gat_aggregate)(const int64_t* s, const int64_t* t, int64_t E, int64_t
     if (!alpha) free(al);
     return 0;
 }
+
+/* Pullback of the edge part above for an upstream dout (C,H,n), with the logit halves el[h,i] = a[1:C,h]·Wx[:,h,i] and
+ * er[h,j] = a[C+1:2C,h]·Wx[:,h,j] as inputs (z_k = el[t_k] + er[s_k]; their chain into a and Wx is linear):
+ *     α = softmax over in-neighbourhoods of leakyrelu(z);   dα_k = <dout[:,h,t_k], Wx[:,h,s_k]>
+ *     T_i = Σ_{k: t_k=i} α_k dα_k;   dz_k = α_k (dα_k − T_{t_k}) · leakyrelu'(z_k)
+ *     del = scatter(+, dz, t);   der = scatter(+, dz, s);   dWx = scatter(+, α .* dout[:,:,t], s)   (edge part only)
+ * Every sum runs in COO edge order.  Only (H,E) temporaries: no (C,H,E) tensor.  alpha (H,E) is optional. */
+int FN(orc_gat_aggregate_bwd)(const int64_t* s, const int64_t* t, int64_t E, int64_t n, const T* Wx, const T* el,
+                              const T* er, int64_t C, int64_t H, T slope, const T* dout, T* dWx, T* del, T* der,
+                              T* alpha) {
+    const size_t EH = (size_t)(E * H > 0 ? E * H : 1);
+    T* u = (T*)malloc(sizeof(T) * EH);
+    T* al = alpha ? alpha : (T*)malloc(sizeof(T) * EH);
+    T* dz = (T*)malloc(sizeof(T) * EH);                 /* α·dα, then dz */
+    T* tn = (T*)malloc(sizeof(T) * (size_t)(n * H > 0 ? n * H : 1));
+    if (!u || !al || !dz || !tn) return 1;
+    for (int64_t k = 0; k < E; ++k)
+        for (int64_t h = 0; h < H; ++h) {
+            const T z = el[(t[k] - 1) * H + h] + er[(s[k] - 1) * H + h];
+            u[k * H + h] = z > 0 ? z : slope * z;
+        }
+    FN(orc_softmax_edge_neighbors)(t, E, n, u, H, al);
+    for (int64_t k = 0; k < E; ++k) {
+        const T* di = dout + (t[k] - 1) * C * H;
+        const T* wj = Wx + (s[k] - 1) * C * H;
+        for (int64_t h = 0; h < H; ++h) {
+            T acc = 0;                                  /* dα = <dout[:,h,t], Wx[:,h,s]>, channel order */
+            for (int64_t c = 0; c < C; ++c) acc = acc + di[h * C + c] * wj[h * C + c];
+            dz[k * H + h] = acc;
+            u[k * H + h] = al[k * H + h] * acc;
+        }
+    }
+    FN(orc_scatter)(ORC_SUM, u, t, E, H, n, tn);        /* T = scatter(+, α .* dα, t) */
+    for (int64_t k = 0; k < E; ++k)
+        for (int64_t h = 0; h < H; ++h) {
+            const T z = el[(t[k] - 1) * H + h] + er[(s[k] - 1) * H + h];
+            dz[k * H + h] = al[k * H + h] * (dz[k * H + h] - tn[(t[k] - 1) * H + h]) * (z > 0 ? (T)1 : slope);
+        }
+    FN(orc_scatter)(ORC_SUM, dz, t, E, H, n, del);
+    FN(orc_scatter)(ORC_SUM, dz, s, E, H, n, der);
+    for (int64_t i = 0; i < n * C * H; ++i) dWx[i] = 0;
+    for (int64_t k = 0; k < E; ++k) {                   /* scatter(+, α .* dout[:,:,t], s) without the (C,H,E) tensor */
+        T* dj = dWx + (s[k] - 1) * C * H;
+        const T* di = dout + (t[k] - 1) * C * H;
+        for (int64_t h = 0; h < H; ++h) {
+            const T w = al[k * H + h];
+            for (int64_t c = 0; c < C; ++c) dj[h * C + c] = dj[h * C + c] + w * di[h * C + c];
+        }
+    }
+    free(u); free(dz); free(tn);
+    if (!alpha) free(al);
+    return 0;
+}

@@ -158,6 +158,36 @@ def gat_aggregate(s, t, n, Wx, a, slope=0.2):
     return out, alpha
 
 
+def gat_logit_halves(Wx, a):
+    """el (N, H), er (N, H): the target and source halves of sum(a .* vcat(Wxi, Wxj), dims=1), in Wx's dtype.
+    Wx (N, H, C) rows, a (H, 2C) rows."""
+    Cc = Wx.shape[2]
+    a = np.asarray(a, dtype=Wx.dtype)
+    return (np.einsum("nhc,hc->nh", Wx, a[:, :Cc]), np.einsum("nhc,hc->nh", Wx, a[:, Cc:]))
+
+
+def gat_aggregate_bwd(s, t, n, Wx, dout, slope=0.2, *, a=None, el=None, er=None):
+    """Pullback of gat_aggregate for the upstream dout (N, H, C).  The logits come from el, er (N, H) or, given a (H, 2C),
+    from gat_logit_halves(Wx, a).  Returns (dWx (N,H,C): the edge part only, del (N,H), der (N,H), alpha (E,H)); the
+    logit chain into Wx and a is dWx += del a[:, :C] + der a[:, C:],  da = [Σ_n del Wx, Σ_n der Wx]."""
+    Wx = np.ascontiguousarray(Wx)
+    if a is not None:
+        el, er = gat_logit_halves(Wx, a)
+    el, er, dout = _f(el, Wx.dtype), _f(er, Wx.dtype), _f(dout, Wx.dtype)
+    s, t = _idx(s), _idx(t)
+    N, H, Cc = Wx.shape
+    assert dout.shape == Wx.shape and el.shape == er.shape == (N, H)
+    dWx = np.empty_like(Wx)
+    del_, der = np.empty((n, H), dtype=Wx.dtype), np.empty((n, H), dtype=Wx.dtype)
+    alpha = np.empty((len(s), H), dtype=Wx.dtype)
+    ct = C.c_float if Wx.dtype == np.float32 else C.c_double
+    rc = getattr(lib(), "orc_gat_aggregate_bwd" + _sfx(Wx.dtype))(
+        _p(s), _p(t), C.c_int64(len(s)), C.c_int64(n), _p(Wx), _p(el), _p(er), C.c_int64(Cc), C.c_int64(H), ct(slope),
+        _p(dout), _p(dWx), _p(del_), _p(der), _p(alpha))
+    assert rc == 0
+    return dWx, del_, der, alpha
+
+
 def add_self_loops(s, t, n):
     s, t = _idx(s), _idx(t)
     s2 = np.empty(len(s) + n, dtype=np.int64)
